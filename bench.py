@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — denoised frames/s of the ray-trace + SVGF hot path on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1,2,3,4,5}] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1,2,3,4,5}] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one frame of the configuration's passes.  --config picks one of BASELINE.json's five configurations as
 SURVEY.md §8d makes them concrete; the default is the largest single-GPU one, config 3:
@@ -298,6 +298,24 @@ def texel_bytes(img):
     return {1: 4, 2: 2, 3: 4, 4: 8, 5: 1}[img.format]
 
 
+DUMP_BYTES = 64 * 10**6  # --dump-outputs: all files together stay below this
+
+
+def dump_outputs(out_dir, images, seed=0):
+    """Writes every image as out_dir/<name>.npy: float32 (float64 for 32-bit integer images), shape (H, W[, C]).  An image larger than
+    its share of DUMP_BYTES is written as a fixed sample of its pixels drawn with `seed`: (n, C), the pixels in row-major order, so two
+    builds given the same arguments write the same pixels."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = (DUMP_BYTES - 4096 * len(images)) // max(1, len(images))  # 4096: room for each .npy header
+    for name, a in images.items():
+        a = a.astype(np.float64 if a.dtype.kind in "iu" and a.dtype.itemsize == 4 else np.float32)
+        if a.nbytes > share:
+            px = a.reshape(a.shape[0] * a.shape[1], -1)
+            n = share // (px.shape[1] * px.itemsize)
+            a = px[np.sort(np.random.default_rng(seed).choice(px.shape[0], n, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------------------- post-pass leg
 def post_leg(W, H, tris):
     """Informational, run in its OWN process by the default single-GPU bench (crash isolation: these kernels had no GPU time before the
@@ -425,7 +443,11 @@ def main():
     ap.add_argument("--config", type=int, default=3, choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the pan / dense-K5 / host-G-buffer legs (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write every pass's final output of the last step as DIR/<pass>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     cfg = CONFIGS[args.config]
     W, H = cfg["W"], cfg["H"]
     rank = int(os.environ.get("RANK", "0"))
@@ -553,6 +575,8 @@ def main():
     rig.stats(stream)  # reset the ray counters
     r_val = timed(step_resident, args.steps, profile=True, sample=True)
     st_val = rig.stats(stream)
+    if args.dump_outputs and rank == 0:  # the final outputs are gathered: rank 0 holds whole frames
+        dump_outputs(args.dump_outputs, {name: p.download(100, stream) for name, p in rig.passes.items()})
     r_dist = None
     if world > 1:
         gather(False)

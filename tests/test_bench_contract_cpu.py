@@ -40,3 +40,22 @@ def test_reference_arm_line(config):
 def test_reference_arm_only_rank0_prints():
     env = {"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2", "MASTER_ADDR": "127.0.0.1", "MASTER_PORT": "29599"}
     assert run_reference(1, env) == []
+
+
+def test_dump_outputs_bounded_and_repeatable(tmp_path):
+    """--dump-outputs: a 4K RGBA16F image is sampled under its share of the 64 MB, a small R32_UINT image is written whole and exactly,
+    and the same images give the same files."""
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(3)
+    imgs = {"big": rng.standard_normal((2160, 3840, 4)).astype(np.float16), "small": rng.integers(0, 2**32, (48, 64), dtype=np.uint32)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), imgs)
+    total = sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a"))
+    assert sorted(os.listdir(tmp_path / "a")) == ["big.npy", "small.npy"] and total <= bench.DUMP_BYTES
+    big, small = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "a" / "small.npy")
+    assert big.dtype == np.float32 and big.shape[1] == 4 and big.nbytes > 0.99 * bench.DUMP_BYTES / 2  # the sample fills its half of the budget
+    assert small.dtype == np.float64 and np.array_equal(small, imgs["small"])
+    assert np.array_equal(big, np.load(tmp_path / "b" / "big.npy"))
+    px = imgs["big"].reshape(-1, 4).astype(np.float32)
+    assert all((px == big[i]).all(1).any() for i in (0, len(big) // 2, -1)), "sampled values are not pixels of the image"

@@ -33,22 +33,6 @@ def _orc_const(name, n=6):
     return [buf[i] for i in range(cnt)]
 
 
-def test_generated_fixture_is_current_when_reference_is_present():
-    """In the build container the committed JSON must be what the script extracts today (on the GPU box: skipped)."""
-    if not os.path.isdir("/root/reference/src/shaders"):
-        pytest.skip("/root/reference not present (GPU box)")
-    import subprocess
-    import sys
-    import tempfile
-    src = open(os.path.join(HERE, "golden", "make_ref_constants.py")).read()
-    with tempfile.TemporaryDirectory() as td:
-        script = os.path.join(td, "make_ref_constants.py")
-        open(script, "w").write(src)
-        subprocess.run([sys.executable, script], check=True, stdout=subprocess.DEVNULL)
-        fresh = json.load(open(os.path.join(td, "ref_constants.json")))
-    assert fresh == REF
-
-
 @pytest.mark.parametrize("side,key", [(16, "gi_border_offsets_depth_16"), (8, "gi_border_offsets_irradiance_8")])
 def test_border_offset_tables_equal_reference(side, key):
     L = O.lib()
