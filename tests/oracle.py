@@ -180,6 +180,7 @@ class ShadowsOracle:
         P.radius, P.filter_iterations, P.feedback_iteration, P.denoise = 1, 4, 1, 1
         self.final = None
         self.band = None  # (b0, b1): emulate a sharded rank — rows a rank would not compute are overwritten with garbage
+        self.halos = (16, 24)  # (denoise, ray trace) rows beyond the band a rank recomputes: hr_shard_halo_rows for the parameters above
         # cooperative ray trace emulation (DESIGN.md §9): this rank traces mask rows [rt_share[0], rt_share[1]) only and
         # mask_exchange(mask, a, b) must return the complete mask (what k_rt_push + the frame ticks do between GPUs)
         self.rt_share, self.mask_exchange = None, None
@@ -218,7 +219,7 @@ class ShadowsOracle:
             if self.rt_share is not None:
                 _coop_mask(self)
             else:
-                self._poison(self.mask, 24, div=4)
+                self._poison(self.mask, self.halos[1], div=4)
             self.final = self.mask
             if not P.denoise:
                 return
@@ -226,7 +227,7 @@ class ShadowsOracle:
                                    P.moments_alpha, p(self.temporal), p(self.moments[pp]), p(self.tile_flags))
         self.cur_moments = self.moments[pp]
         for a in (self.temporal, self.moments[pp], self.tile_flags):
-            self._poison(a, 16, div=8 if a is self.tile_flags else 1)
+            self._poison(a, self.halos[0], div=8 if a is self.tile_flags else 1)
         ping = False
         src = self.temporal
         for i in range(P.filter_iterations):
@@ -234,7 +235,7 @@ class ShadowsOracle:
             power = P.power if i == P.filter_iterations - 1 else 0.0
             L.orc_shadows_atrous(C.byref(gc), p(src), p(self.tile_flags), P.radius, 1 << i, P.phi_visibility, P.phi_normal, P.sigma_depth, power,
                                  p(self.atrous[write_idx]))
-            self._poison(self.atrous[write_idx], 16)
+            self._poison(self.atrous[write_idx], self.halos[0])
             ping = not ping
             if P.feedback_iteration == i:
                 self.prev_image[:] = self.atrous[write_idx]

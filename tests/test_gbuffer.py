@@ -64,8 +64,11 @@ def test_motion_vectors_are_zero_for_a_static_camera_and_nonzero_under_pan():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("scene_kind,tris", [(pyhr.SCENE_SHADOWS_TEST, 0), (pyhr.SCENE_ARCADE, 20000)])
-def test_device_gbuffer_is_bit_exact_against_the_oracle(scene_kind, tris):
+@pytest.mark.parametrize("scene_kind,tris,W,H", [pytest.param(pyhr.SCENE_SHADOWS_TEST, 0, W, H, id=f"{pyhr.SCENE_SHADOWS_TEST}-0"),
+                                                 pytest.param(pyhr.SCENE_ARCADE, 20000, W, H, id=f"{pyhr.SCENE_ARCADE}-20000"),
+                                                 # odd width, H % 4 != 0: partial curvature quads at the right / bottom edge, mips 101x58 and 50x29
+                                                 pytest.param(pyhr.SCENE_ARCADE, 20000, 203, 117, id=f"{pyhr.SCENE_ARCADE}-20000-203x117")])
+def test_device_gbuffer_is_bit_exact_against_the_oracle(scene_kind, tris, W, H):
     sc = pyhr.SynthScene(scene_kind, tris)
     ss = O.ShadingScene(sc, brute=False)
     ctx = pyhr.Context(0)

@@ -37,7 +37,9 @@ def close(a, b, name, r=1e-3, m=6e-3):
     assert d.max() <= m, f"{name}: max abs {d.max()}"
 
 
-def run(scene_kind, n_frames, refl_scale, with_ddgi, light=None, cam=None, pan_from=None, tris=0):
+def run(scene_kind, n_frames, refl_scale, with_ddgi, light=None, cam=None, pan_from=None, tris=0, W=W, H=H, params=None, record=None):
+    """params: hr_reflections_params fields to override (the oracle reads the same structure); record: a list that receives
+    the device a-trous and final images of every frame"""
     sc = pyhr.SynthScene(scene_kind, tris)
     ss = O.ShadingScene(sc, brute=sc.n_tris <= 4096)
     bn = pyhr.blue_noise()
@@ -51,6 +53,8 @@ def run(scene_kind, n_frames, refl_scale, with_ddgi, light=None, cam=None, pan_f
     rf = pyhr.ReflectionsPass(ctx, W, H, refl_scale)
     for P in ([dd.params] if dd else []) + [rf.params]:
         P.sky_color[0], P.sky_color[1], P.sky_color[2] = SKY
+    for k, v in (params or {}).items():
+        setattr(rf.params, k, v)
     odd = None
     if dd:
         dd.params.probe_distance = 4.0 if scene_kind == pyhr.SCENE_SHADOWS_TEST else 12.0
@@ -94,6 +98,8 @@ def run(scene_kind, n_frames, refl_scale, with_ddgi, light=None, cam=None, pan_f
         close(mo_c, mo_o, f"frame {i} reflections moments")
         close(f16(rf.download(2)), O.h2f(orf.atrous_out), f"frame {i} reflections a-trous")
         close(f16(rf.download(100)), O.h2f(orf.final), f"frame {i} reflections final")
+        if record is not None:
+            record.append((rf.download(2), rf.download(100)))
     stats = (float(rt_o[..., :3].mean()), float((rt_o[..., 3] > 0).mean()))
     rf.destroy()
     if dd:

@@ -25,7 +25,7 @@ SH = dict(temporal=1, atrous=2, moments=4, prev=5, final=100)
 AO = dict(temporal=1, blur=2, length=4, final=100)
 
 
-def frames(n, pan_from=3, vertical=0.0):
+def frames(n, pan_from=3, vertical=0.0, W=W, H=H):
     f = None
     for i in range(n):
         dx = 0.0 if i < pan_from else 0.05 * (i - pan_from + 1)
@@ -34,7 +34,7 @@ def frames(n, pan_from=3, vertical=0.0):
         yield f
 
 
-def make_rank(device, sc, sh_scale, ao_scale, rank=0, world=1):
+def make_rank(device, sc, sh_scale, ao_scale, rank=0, world=1, W=W, H=H):
     c = pyhr.Context(device)
     c.set_bluenoise(*pyhr.blue_noise())
     c.build_scene(sc)
@@ -83,11 +83,14 @@ def test_sharded_emulation_bit_identical(world, sh_scale, ao_scale):
         c.close()
 
 
-@pytest.mark.parametrize("world,sh_scale,ao_scale", [(2, 0, 1), (5, 0, 0), (8, 1, 1)])
-def test_peer_history_emulation_bit_identical(world, sh_scale, ao_scale):
+# 203x117 (world 3): odd pass widths, a last band that ends in a partial tile, and an odd full-res height for the upsample rows
+# of the last band (b1 >= H ? H0)
+@pytest.mark.parametrize("world,sh_scale,ao_scale,W,H", [pytest.param(2, 0, 1, W, H, id="2-0-1"), pytest.param(5, 0, 0, W, H, id="5-0-0"),
+                                                         pytest.param(8, 1, 1, W, H, id="8-1-1"), pytest.param(3, 1, 1, 203, 117, id="3-1-1-203x117")])
+def test_peer_history_emulation_bit_identical(world, sh_scale, ao_scale, W, H):
     sc = pyhr.SynthScene(pyhr.SCENE_SHADOWS_TEST)
-    ref = make_rank(0, sc, sh_scale, ao_scale)
-    ranks = [make_rank(0, sc, sh_scale, ao_scale, r, world) for r in range(world)]
+    ref = make_rank(0, sc, sh_scale, ao_scale, W=W, H=H)
+    ranks = [make_rank(0, sc, sh_scale, ao_scale, r, world, W, H) for r in range(world)]
     for r in range(world):
         for q in range(world):
             if q != r:
@@ -98,7 +101,7 @@ def test_peer_history_emulation_bit_identical(world, sh_scale, ao_scale):
     # cost-balanced share of the whole image and pushes it to all peers), so the emulated ranks must be able to run
     # concurrently: one CUDA stream per rank (conftest.py raises CUDA_DEVICE_MAX_CONNECTIONS so they get separate queues).
     streams = [torch.cuda.Stream() for _ in range(world)]
-    for f in frames(8, pan_from=2, vertical=0.35):
+    for f in frames(8, pan_from=2, vertical=0.35, W=W, H=H):
         g = pyhr.write_gbuffer(sc, f, W, H)
         ref[0].gbuffer_upload(f.ping_pong, g)
         ref[1].render(f)
@@ -190,7 +193,7 @@ def test_nccl_sharded_matches_single(tmp_path):
 RF = dict(rt=0, temporal=1, atrous=2, moments=4, final=100)
 
 
-def _refl_rank(device, sc, scale, rank=0, world=1):
+def _refl_rank(device, sc, scale, rank=0, world=1, W=W, H=H):
     c = pyhr.Context(device)
     c.set_bluenoise(*pyhr.blue_noise())
     c.build_scene(sc)
@@ -202,21 +205,22 @@ def _refl_rank(device, sc, scale, rank=0, world=1):
     return c, p
 
 
-@pytest.mark.parametrize("world,scale", [(2, 0), (5, 1), (8, 0)])
-def test_peer_history_emulation_reflections(world, scale):
+@pytest.mark.parametrize("world,scale,W,H", [pytest.param(2, 0, W, H, id="2-0"), pytest.param(5, 1, W, H, id="5-1"), pytest.param(8, 0, W, H, id="8-0"),
+                                             pytest.param(3, 1, 203, 117, id="3-1-203x117")])
+def test_peer_history_emulation_reflections(world, scale, W, H):
     """N linked ranks on one GPU (the production multi-GPU data path minus CUDA IPC): every rank traces the 8-row chunks
     c % world == rank of the whole image and pushes them to the ranks that filter those rows; reprojection pulls history
     texels from the owner of their row.  Each rank's band of every stage must be BIT-IDENTICAL to the single-GPU images."""
     sc = pyhr.SynthScene(pyhr.SCENE_SHADOWS_TEST)
-    ref = _refl_rank(0, sc, scale)
-    ranks = [_refl_rank(0, sc, scale, r, world) for r in range(world)]
+    ref = _refl_rank(0, sc, scale, W=W, H=H)
+    ranks = [_refl_rank(0, sc, scale, r, world, W, H) for r in range(world)]
     for r in range(world):
         for q in range(world):
             if q != r:
                 ranks[r][1].link_local(q, ranks[q][1])
     streams = [torch.cuda.Stream() for _ in range(world)]
     ph = H >> scale
-    for f in frames(7, pan_from=2, vertical=0.35):
+    for f in frames(7, pan_from=2, vertical=0.35, W=W, H=H):
         g = pyhr.write_gbuffer(sc, f, W, H)
         ref[0].gbuffer_upload(f.ping_pong, g)
         ref[1].render(f, None)

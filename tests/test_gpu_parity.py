@@ -35,7 +35,9 @@ def camera_path(i, pan_from=None):
     return (dx, 14.0, 34.0), (dx, 3.0, 0.0)
 
 
-def run_sequence(ctx, scene_kind, W, H, n_frames, sh_scale, ao_scale, pan_from=None, visible_kind=None, cam=None, check=None, light=None):
+def run_sequence(ctx, scene_kind, W, H, n_frames, sh_scale, ao_scale, pan_from=None, visible_kind=None, cam=None, check=None, light=None, sh_params=None,
+                 ao_params=None):
+    """sh_params / ao_params: hr_shadows_params / hr_ao_params fields to override, on the device pass and the oracle alike"""
     bn = pyhr.blue_noise()
     sc = pyhr.SynthScene(scene_kind)
     vis_sc = sc if visible_kind is None else pyhr.SynthScene(visible_kind)
@@ -46,6 +48,10 @@ def run_sequence(ctx, scene_kind, W, H, n_frames, sh_scale, ao_scale, pan_from=N
     # fresh g-buffer per sequence: recreate the context-level buffers by using a new context when the size changes
     sh, ao = pyhr.Pass(ctx, "shadows", W, H, sh_scale), pyhr.Pass(ctx, "ao", W, H, ao_scale)
     osh, oao = O.ShadowsOracle(W, H, sh_scale), O.AOOracle(W, H, ao_scale)
+    for over, passes in ((sh_params, (sh, osh)), (ao_params, (ao, oao))):
+        for k, v in (over or {}).items():
+            for x in passes:
+                setattr(x.params, k, v)
     f, prev_g = None, O.zero_gbuf_mips(W, H)
     # the device history slot must start as zeros too
     zero = pyhr.GBufferHost(W, H)
@@ -212,17 +218,22 @@ def test_trace_random_rays_vs_bruteforce(ctx_256):
     L.hr_scene_destroy(h)
 
 
-def test_gbuffer_mips_match_oracle(ctx_256):
+def check_gbuffer_mips(ctx, W0, H0):
+    """host G-buffer of the shadows-test scene uploaded at W0 x H0: the device mips 0-2 equal the oracle's bit for bit"""
     sc = pyhr.SynthScene(pyhr.SCENE_SHADOWS_TEST)
-    f = pyhr.make_frame((0, 14, 34), (0, 3, 0), 256, 144)
-    g = pyhr.write_gbuffer(sc, f, 256, 144)
-    ctx_256.gbuffer_upload(0, g)
+    f = pyhr.make_frame((0, 14, 34), (0, 3, 0), W0, H0)
+    g = pyhr.write_gbuffer(sc, f, W0, H0)
+    ctx.gbuffer_upload(0, g)
     om = O.GBufMips(g)
     for mip in range(3):
         W, H, gb2, gb3, d = om.levels[mip]
-        assert np.array_equal(ctx_256.gbuffer_download(0, mip, 2, 256, 144), gb2)
-        assert np.array_equal(ctx_256.gbuffer_download(0, mip, 3, 256, 144), gb3)
-        assert np.array_equal(ctx_256.gbuffer_download(0, mip, 0, 256, 144), d)
+        assert np.array_equal(ctx.gbuffer_download(0, mip, 2, W0, H0), gb2), f"mip {mip} ({W}x{H}) gb2"
+        assert np.array_equal(ctx.gbuffer_download(0, mip, 3, W0, H0), gb3), f"mip {mip} ({W}x{H}) gb3"
+        assert np.array_equal(ctx.gbuffer_download(0, mip, 0, W0, H0), d), f"mip {mip} ({W}x{H}) depth"
+
+
+def test_gbuffer_mips_match_oracle(ctx_256):
+    check_gbuffer_mips(ctx_256, 256, 144)
 
 
 def test_atrous_tiled_equals_naive_and_oracle_1080p():

@@ -55,7 +55,8 @@ def _gather_bands(dist, arr, pass_h, rank, world, shift=0):
     return out
 
 
-def _worker(rank, world, port, q):
+def _worker(rank, world, port, q, W=W, H=H, radius=1, iters=4):
+    """radius / iters: shadows a-trous parameters; the ranks recompute the halos hr_shard_halo_rows derives from them"""
     import torch.distributed as dist
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
@@ -67,6 +68,9 @@ def _worker(rank, world, port, q):
         bn = pyhr.blue_noise()
         ref_sh, ref_ao = O.ShadowsOracle(W, H, 0), O.AOOracle(W, H, 1)
         sh, ao = O.ShadowsOracle(W, H, 0), O.AOOracle(W, H, 1)
+        for o in (ref_sh, sh):
+            o.params.radius, o.params.filter_iterations = radius, iters
+        sh.halos = pyhr.shard_halo_rows("shadows", radius, iters)
         sh.band = shard_rows(sh.H, rank, world)
         ao.band = shard_rows(ao.H, rank, world)
         f, prev = None, O.zero_gbuf_mips(W, H)
@@ -241,12 +245,12 @@ def _worker_refl(rank, world, port, q):
         dist.destroy_process_group()
 
 
-def _run_world(worker, world):
+def _run_world(worker, world, *args):
     import torch.multiprocessing as mp
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
-    port = 29500 + os.getpid() % 2000 + world + (17 if worker is _worker_coop else 0) + (41 if worker is _worker_refl else 0)
-    procs = [ctx.Process(target=worker, args=(r, world, port, q)) for r in range(world)]
+    port = 29500 + os.getpid() % 2000 + world + (17 if worker is _worker_coop else 0) + (41 if worker is _worker_refl else 0) + (67 if worker is _worker else 0)
+    procs = [ctx.Process(target=worker, args=(r, world, port, q) + args) for r in range(world)]
     for p_ in procs:
         p_.start()
     res = [q.get(timeout=600) for _ in range(world)]
@@ -273,6 +277,13 @@ def test_sharded_oracle_gloo(world):
     for p_ in procs:
         p_.join(60)
     assert res == ["ok"] * world, res
+
+
+@pytest.mark.parametrize("radius,iters", [(2, 6), (2, 2)])
+def test_sharded_oracle_ragged_param_halos_gloo(radius, iters):
+    """203x117 on 3 ranks: the last band ends in a partial tile (rows 80..117) and the shadows halos come from hr_shard_halo_rows
+    for a-trous parameters off the defaults (radius 2 with 6 iterations: 128 rows, the whole image; with 2 iterations: 8 rows)"""
+    assert _run_world(_worker, 3, 203, 117, radius, iters) == ["ok"] * 3
 
 
 @pytest.mark.parametrize("world", [2, 3])
